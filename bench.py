@@ -73,6 +73,41 @@ def make_network(device):
     return net.to(device) if device is not None else net
 
 
+# --dump-outputs: larger arrays are cut to a fixed, seeded sample of their elements.  The cap keeps the learned 784 x 1600
+# weights of the metric configuration whole and c3 (batch 256, n = 6400, two 6400 x 6400 static matrices) under 64 MB
+DUMP_MAX_ELEMS = 5 << 18
+DUMP_MAX_BYTES = 64 << 20   # --dump-outputs: all files together
+
+
+def dump_outputs(path: str, net) -> None:
+    """--dump-outputs: what a caller of Network.run reads after the last timed window — every layer's spikes, voltages,
+    traces, adaptive thresholds and refractory counters and every connection's weights — as float32 DIR/<name>.npy, so
+    that two builds can be compared output for output.  An array of more than DUMP_MAX_ELEMS elements is flattened and
+    cut to the same seeded sample of positions on every run."""
+    import numpy as np
+    import torch
+
+    arrays = {}
+    for lname, layer in net.layers.items():
+        for var in ("s", "v", "x", "theta", "refrac_count"):
+            val = getattr(layer, var, None)
+            if isinstance(val, torch.Tensor) and val.numel():
+                arrays[f"{lname}.{var}"] = val
+    for (src, tgt), conn in net.connections.items():
+        arrays[f"{src}-{tgt}.w"] = conn.w
+    for name, val in arrays.items():
+        a = val.detach().float().cpu().numpy()
+        if a.size > DUMP_MAX_ELEMS:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        arrays[name] = a
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:   # checked before anything is written: no partial DIR
+        raise ValueError(f"--dump-outputs: {total / 2**20:.1f} MB of outputs, more than {DUMP_MAX_BYTES >> 20} MB")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 class ClockSampler:
     """Samples nvidia-smi clocks / throttle reasons during the timed region (B200_PROFILING.md)."""
 
@@ -307,7 +342,7 @@ def run_config4(args) -> None:
         net.add_connection(topology.Connection(H, O, update_rule=MSTDP, nu=1e-2, reduction=torch.sum, wmin=-1.0, wmax=1.0), "H", "O")
         return net.to(device) if device is not None else net
 
-    K, W = min(args.steps, 5), min(max(args.warmup, 1), 2)
+    K, W = args.steps, min(max(args.warmup, 1), 2)
     g = torch.Generator().manual_seed(11)
     if args.impl == "reference":
         from oracle.oracle import OracleBackend
@@ -357,6 +392,8 @@ def run_config4(args) -> None:
     ms = e0.elapsed_time(e1) / K
     launches = _backend.launches_total - l0
     net.check_errors()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, net)
     # end to end: pinned host spikes in, the output layer's spikes of the last step out, every window
     xdev = torch.empty_like(resident[0])
     out_host = torch.empty(B, 10, dtype=torch.bool).pin_memory()
@@ -401,7 +438,9 @@ def main():
     quiet_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=320, help="timed windows (default: 320 windows = a timed region of >= 0.5 s at the metric configuration)")
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed windows (default: 320 = a timed region of >= 0.5 s at the metric configuration; 5 for c4, "
+                         "which also runs its end-to-end loop and reference arm for that many windows)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--tier", type=int, default=0, help="0 auto, 1 generic kernel, 2 fused DC2015 kernel v1 (grid barrier), 3 fused DC2015 kernel v2 (message exchange)")
@@ -409,7 +448,16 @@ def main():
     ap.add_argument("--config", default="metric", choices=["metric", "c3", "c4"],
                     help="metric: the configuration BASELINE.json's metric is quoted on (DiehlAndCook2015 n=1600, B=128; default); "
                          "c3: configs[2] (n=6400, B=256); c4: configs[3] (conv 32x32 -> 16ch -> 10, MSTDP, 500 timesteps, B=128)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed windows, write the network state the last one left (spikes, voltages, traces, "
+                         "thresholds, weights) to DIR/<name>.npy as float32; the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 5 if args.config == "c4" else 320
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; it does not apply to --impl reference")
     apply_config(args.config)
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.config == "c4":
@@ -475,6 +523,8 @@ def main():
     kern_ms = [a.elapsed_time(b) for a, b in _backend.kernel_events]
     _backend.kernel_events = None
     net.check_errors()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, net)   # before the passes below run the same network again
     value = world * BATCH * T_STEPS * K / (ms_total * 1e-3)
 
     # ---- the FIRST window of a fresh network (W0 as initialised, theta = 0: every neuron still fires easily, so the

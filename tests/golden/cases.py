@@ -14,8 +14,8 @@ import torch
 
 
 def namespace(kind: str) -> SimpleNamespace:
-    """``kind`` = "reference" (live /root/reference via the stub package of SURVEY.md §8c) or
-    "b200" (this repo)."""
+    """``kind`` = "reference" (the original package via the stub package of SURVEY.md §8c: the checkout named by
+    ``BINDSNET_REFERENCE``, else the install baseline/install_ref.sh made under baseline/_ref) or "b200" (this repo)."""
     if kind == "b200":
         import bindsnet_b200 as pkg
         from bindsnet_b200 import encoding, learning, models
@@ -28,12 +28,11 @@ def namespace(kind: str) -> SimpleNamespace:
             import os
 
             here = os.path.dirname(os.path.abspath(__file__))
-            # the live reference: /root/reference in the build container, else the copy baseline/install_ref.sh made
-            ref = "/root/reference/bindsnet"
-            if not os.path.isdir(ref):
+            ref = os.path.join(os.environ.get("BINDSNET_REFERENCE", ""), "bindsnet")
+            if "BINDSNET_REFERENCE" not in os.environ or not os.path.isdir(ref):
                 ref = os.path.join(here, "..", "..", "baseline", "_ref", "bindsnet")
             if not os.path.isdir(ref):
-                raise ImportError("the reference is neither at /root/reference nor under baseline/_ref")
+                raise ImportError("the reference is neither at $BINDSNET_REFERENCE/bindsnet nor under baseline/_ref")
             pkg = types.ModuleType("bindsnet")
             pkg.__path__ = [ref]
             sys.modules["bindsnet"] = pkg

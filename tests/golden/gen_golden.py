@@ -1,7 +1,7 @@
-"""Generate the golden fixtures by running the LIVE reference (/root/reference) under fixed
-seeds.  Run in the build container only (the reference does not exist on the GPU box):
+"""Generate the golden fixtures by running the LIVE reference (the original package, found as
+``cases.namespace("reference")`` finds it) under fixed seeds:
 
-    python tests/golden/gen_golden.py [case ...]
+    BINDSNET_REFERENCE=/path/to/bindsnet-checkout python tests/golden/gen_golden.py [case ...]
 
 For every case of ``cases.py`` this writes ``tests/golden/<case>.npz`` holding the exact input
 spikes (bit-packed), the final state of every layer and connection after ``network.run`` and
@@ -111,7 +111,7 @@ def patch_reference_conv_mstdp(ns) -> None:
     last line views the new eligibility as ``w.size()`` (:2013) — that raises for B > 1 and, for B = 1, makes
     the next step sum over the OUTPUT CHANNELS instead of the batch.  The goldens are produced by the
     reference's own code with that one view taken per sample (the source is re-executed from
-    /root/reference at run time, nothing is copied)."""
+    the reference's own source at run time, nothing is copied)."""
     import inspect
     import textwrap
 

@@ -291,8 +291,9 @@ def test_mstdp_rule_state_and_eligibility_view():
 
 def test_local_connection_structure_matches_the_reference():
     """LocalConnection (topology.py:1304-1484): receptive-field structure (mask of the default initialisation), kernel-scaled
-    norm and the bias the reference always creates — compared with the live reference where it is available."""
+    norm and the bias the reference always creates — compared with the reference's (stored under tests/golden/live)."""
     from bindsnet_b200.network.topology import LocalConnection
+    from live import REF, stored
 
     X, Y = Input(n=64, traces=True), LIFNodes(n=2 * 36, traces=True)
     c = LocalConnection(X, Y, kernel_size=3, stride=1, n_filters=2, norm=0.5, wmin=0.0, wmax=1.0)
@@ -300,21 +301,20 @@ def test_local_connection_structure_matches_the_reference():
     assert int((~c.mask).sum()) == 2 * 36 * 9                       # n_filters * conv_prod * kernel_prod weights inside the fields
     assert torch.all(c.w[c.mask] == 0) and float(c.norm) == pytest.approx(0.5 * 9)
     assert bool(((~c.mask).sum(0) == 9).all())                      # every target neuron sees exactly one 3x3 field
-    try:
-        import cases
-        ref = cases.namespace("reference")
-    except Exception:
-        return
-    rx, ry = ref.nodes.Input(n=64, traces=True), ref.nodes.LIFNodes(n=72, traces=True)
-    rc = ref.topology.LocalConnection(rx, ry, kernel_size=3, stride=1, n_filters=2, norm=0.5, wmin=0.0, wmax=1.0)
-    assert torch.equal(rc.mask.bool(), c.mask.bool()) and torch.equal(rc.locations, c.locations)
-    assert float(rc.norm) == pytest.approx(float(c.norm))
+    def reference():
+        rx, ry = REF.nodes.Input(n=64, traces=True), REF.nodes.LIFNodes(n=72, traces=True)
+        rc = REF.topology.LocalConnection(rx, ry, kernel_size=3, stride=1, n_filters=2, norm=0.5, wmin=0.0, wmax=1.0)
+        rc2 = REF.topology.LocalConnection(REF.nodes.Input(n=48, traces=True), REF.nodes.LIFNodes(n=27, traces=True), kernel_size=(2, 4),
+                                           stride=(2, 2), n_filters=3, input_shape=(6, 8))
+        return rc.mask.bool(), rc.locations, float(rc.norm), rc2.mask.bool(), rc2.locations
+
+    mask, locations, norm, mask2, locations2 = stored("structure", reference)
+    assert torch.equal(mask, c.mask.bool()) and torch.equal(locations, c.locations)
+    assert norm == pytest.approx(float(c.norm))
     # rectangular input, stride 2
     X2, Y2 = Input(n=6 * 8, traces=True), LIFNodes(n=3 * 3 * 3, traces=True)
     c2 = LocalConnection(X2, Y2, kernel_size=(2, 4), stride=(2, 2), n_filters=3, input_shape=(6, 8))
-    rc2 = ref.topology.LocalConnection(ref.nodes.Input(n=48, traces=True), ref.nodes.LIFNodes(n=27, traces=True), kernel_size=(2, 4),
-                                       stride=(2, 2), n_filters=3, input_shape=(6, 8))
-    assert torch.equal(rc2.locations, c2.locations) and torch.equal(rc2.mask.bool(), c2.mask.bool())
+    assert torch.equal(locations2, c2.locations) and torch.equal(mask2, c2.mask.bool())
 
 
 def test_boosted_lif_and_mcculloch_pitts_state_like_reference():

@@ -1,8 +1,8 @@
 """``models.IncreasingInhibitionNetwork`` (reference: models.py:349-454) and ``models.LocallyConnectedNetwork``
-(:457-584): same wiring as the live reference (static weights equal to the bit, same layer / connection parameters), and
-a learning window through the live reference — ``torch.multinomial`` replaced by the shared tie-break hash, like the
-goldens — equals ours on the oracle; the kernels' CUDA sources on the emulation of tests/emu agree with the oracle bit
-for bit.  CPU only; skipped where the reference is absent."""
+(:457-584): same wiring as the reference (static weights equal to the bit, same layer / connection parameters), and
+a learning window through the reference — ``torch.multinomial`` replaced by the shared tie-break hash, like the
+goldens — equals ours on the oracle (the reference's side stored under tests/golden/live); the kernels' CUDA sources on
+the emulation of tests/emu agree with the oracle bit for bit.  CPU only."""
 import os
 import sys
 
@@ -12,17 +12,12 @@ import torch
 
 import cases
 import helpers
+from live import REF, stored
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "emu"))
 sys.path.insert(0, os.path.join(HERE, "golden"))
 
-try:
-    REF = cases.namespace("reference")
-except Exception:  # pragma: no cover
-    REF = None
-
-pytestmark = pytest.mark.skipif(REF is None, reason="live reference not available")
 T, B, SEED = 60, 3, 515
 
 
@@ -50,22 +45,36 @@ def _make(ns, which):
 
 @pytest.mark.parametrize("which", ["increasing", "local"])
 def test_wiring_equals_the_live_reference(which):
-    ref, _ = _make(REF, which)
+    params = ("thresh", "rest", "reset", "refrac", "tc_decay", "tc_trace", "theta_plus", "tc_theta_decay")
+
+    def reference():
+        ref, _ = _make(REF, which)
+        a = ref.connections[("X", "Y")]
+        out = {"layers": list(ref.layers), "connections": list(ref.connections), "Y->Y/w": ref.connections[("Y", "Y")].w,
+               "Y": {name: float(getattr(ref.layers["Y"], name)) for name in params},
+               "X->Y": (float(a.wmin), float(a.wmax), float(a.norm)), "nu": [float(v) for v in a.update_rule.nu]}
+        if which == "local":
+            out["mask"], out["locations"] = a.mask, a.locations
+        else:
+            out["n_sqrt"] = ref.n_sqrt
+        return out
+
+    ref = stored("wiring", reference)
     ours, _ = _make(cases.namespace("b200"), which)
-    assert list(ref.layers) == list(ours.layers) and list(ref.connections) == list(ours.connections)
-    assert torch.equal(ref.connections[("Y", "Y")].w, ours.connections[("Y", "Y")].w)
-    for name in ("thresh", "rest", "reset", "refrac", "tc_decay", "tc_trace", "theta_plus", "tc_theta_decay"):
-        assert float(getattr(ref.layers["Y"], name)) == float(getattr(ours.layers["Y"], name)), name
-    a, b = ref.connections[("X", "Y")], ours.connections[("X", "Y")]
-    assert (float(a.wmin), float(a.wmax), float(a.norm)) == (float(b.wmin), float(b.wmax), float(b.norm))
-    assert [float(v) for v in a.update_rule.nu] == [float(v) for v in b.update_rule.nu]
+    assert ref["layers"] == list(ours.layers) and ref["connections"] == list(ours.connections)
+    assert torch.equal(ref["Y->Y/w"], ours.connections[("Y", "Y")].w)
+    for name in params:
+        assert ref["Y"][name] == float(getattr(ours.layers["Y"], name)), name
+    b = ours.connections[("X", "Y")]
+    assert ref["X->Y"] == (float(b.wmin), float(b.wmax), float(b.norm))
+    assert ref["nu"] == [float(v) for v in b.update_rule.nu]
     if which == "local":
-        assert torch.equal(a.mask, b.mask) and torch.equal(a.locations, b.locations)
+        assert torch.equal(ref["mask"], b.mask) and torch.equal(ref["locations"], b.locations)
         # a freshly drawn weight matrix lives inside the same receptive fields, within the same bounds
         fresh = cases.namespace("b200").models.LocallyConnectedNetwork(64, [8, 8], 4, 2, 3).connections[("X", "Y")]
         assert torch.equal(fresh.w == 0, b.mask) and float(fresh.w.max()) <= 1.0
     else:
-        assert ours.n_sqrt == ref.n_sqrt == 5
+        assert ours.n_sqrt == ref["n_sqrt"] == 5
 
 
 @pytest.mark.parametrize("which", ["increasing", "local"])
@@ -73,19 +82,22 @@ def test_learning_window_matches_the_live_reference(which):
     from gen_golden import OneSpikePatch
     from oracle.oracle import OracleBackend
 
-    ref, x = _make(REF, which)
-    rmon = REF.monitors.Monitor(ref.layers["Y"], ["s"], time=T); ref.add_monitor(rmon, "Y")
-    with OneSpikePatch(ref, SEED):
-        ref.run(inputs={"X": x.clone()}, time=T)
+    def reference():
+        ref, x = _make(REF, which)
+        rmon = REF.monitors.Monitor(ref.layers["Y"], ["s"], time=T); ref.add_monitor(rmon, "Y")
+        with OneSpikePatch(ref, SEED):
+            ref.run(inputs={"X": x.clone()}, time=T)
+        return rmon.get("s").reshape(T, _batch(which), -1).sum(dim=(0, 1)).numpy(), helpers.snapshot(ref)
+
+    counts, a = stored("window", reference)
     ours, x2 = _make(cases.namespace("b200"), which)
     helpers.add_spike_monitors(ours, T)
     with OracleBackend() as ob:
         ours.run(inputs={"X": x2}, time=T, one_spike_seed=SEED)
         assert ob.err == 0
-    counts = rmon.get("s").reshape(T, _batch(which), -1).sum(dim=(0, 1)).numpy()
     assert counts.sum() > 10, "the window produced no activity: nothing tested"
     assert np.array_equal(counts, helpers.spike_counts(ours, T)["L/Y/count"])
-    a, b = helpers.snapshot(ref), helpers.snapshot(ours)
+    b = helpers.snapshot(ours)
     assert a.keys() == b.keys()
     for k in a:
         if k.endswith("/s"):

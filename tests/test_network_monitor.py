@@ -1,7 +1,8 @@
 """``monitors.NetworkMonitor`` (reference: monitors.py:127-329): per-step recordings of every layer's and connection's
-state variables — growing (``time=None``) and rolling (``time=T``) — equal the live reference's on the same run (spikes
-exactly, voltages and weights within the north_star's tolerances); the same run on the kernels' CUDA sources (emulation
-of tests/emu) equals the oracle bit for bit; ``save`` writes the reference's npz keys.  CPU only."""
+state variables — growing (``time=None``) and rolling (``time=T``) — equal the reference's on the same run (spikes
+exactly, voltages and weights within the north_star's tolerances; the reference's recordings are stored under
+tests/golden/live); the same run on the kernels' CUDA sources (emulation of tests/emu) equals the oracle bit for bit;
+``save`` writes the reference's npz keys.  CPU only."""
 import os
 import sys
 
@@ -10,13 +11,9 @@ import pytest
 import torch
 
 import cases
+from live import REF, stored
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "emu"))
-
-try:
-    REF = cases.namespace("reference")
-except Exception:  # pragma: no cover
-    REF = None
 
 T, B = 30, 2
 
@@ -46,12 +43,11 @@ def _record(ns, time, backend=None):
     return mon
 
 
-@pytest.mark.skipif(REF is None, reason="live reference not available")
 @pytest.mark.parametrize("time", [None, T, 7])
 def test_network_monitor_matches_the_live_reference(time):
     from oracle.oracle import OracleBackend
 
-    ref = _record(REF, time).get()
+    ref = stored("recording", lambda: _record(REF, time).get())
     ours = _record(cases.namespace("b200"), time, OracleBackend).get()
     assert list(ref) == list(ours) == ["X", "Y", ("X", "Y")]
     for key in ref:
@@ -89,7 +85,6 @@ def test_network_monitor_on_the_emulated_kernel_bit_exact_vs_oracle(tmp_path):
     assert list(rolling.get()) == ["Y"] and list(rolling.get()["Y"]) == ["s"] and rolling.get()["Y"]["s"].shape == (5, B, 12)
 
 
-@pytest.mark.skipif(REF is None, reason="live reference not available")
 def test_get_inputs_matches_the_live_reference():
     """``Network._get_inputs`` (network.py:211-250) as a host call: per-target sums of ``compute`` over the connections."""
     from oracle.oracle import OracleBackend
@@ -106,8 +101,7 @@ def test_get_inputs_matches_the_live_reference():
             net.layers[name].s = torch.bernoulli(p * torch.ones(B, net.layers[name].n), generator=g).bool()
         return net
 
-    ref = build(REF)
-    a = ref._get_inputs()
+    a = stored("inputs", lambda: build(REF)._get_inputs())
     ours = build(cases.namespace("b200"))
     with OracleBackend():
         b = ours._get_inputs()

@@ -1,8 +1,9 @@
 """Randomised parity: small networks drawn from a seeded generator (layer kinds, rules, reductions, options, batch
-sizes) run through the LIVE reference and through our host API on the oracle; both must agree within the north_star's
+sizes) run through the reference and through our host API on the oracle; both must agree within the north_star's
 tolerances (final spikes equal, weights 1e-4 relative, state fp32 tolerance, spike counts equal).  The golden fixtures
-pin hand-picked cases; this walks the option space between them.  CPU only; skipped where the reference is absent
-(it is at /root/reference in the build container and under baseline/_ref after baseline/install_ref.sh)."""
+pin hand-picked cases; this walks the option space between them.  The reference's results are stored under
+tests/golden/live (see tests/golden/live.py).  CPU only."""
+import hashlib
 import os
 import sys
 
@@ -12,15 +13,9 @@ import torch
 
 import cases
 import helpers
+from live import REF, stored
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-
-try:
-    REF = cases.namespace("reference")
-except Exception:  # pragma: no cover
-    REF = None
-
-pytestmark = pytest.mark.skipif(REF is None, reason="live reference not available")
 
 NODE_KINDS = ["LIFNodes", "IFNodes", "BoostedLIFNodes", "CurrentLIFNodes", "AdaptiveLIFNodes", "DiehlAndCookNodes", "McCullochPitts"]
 RULES = ["PostPre", "WeightDependentPostPre", "Hebbian", "NoOp"]
@@ -100,31 +95,39 @@ def _snapshot(net):
     return out
 
 
+def _digest(x: torch.Tensor) -> str:
+    return f"{x.dtype} {tuple(x.shape)} " + hashlib.sha256(x.contiguous().numpy().tobytes()).hexdigest()
+
+
 @pytest.mark.parametrize("seed", list(range(24)))
 def test_random_network_oracle_matches_live_reference(seed):
     from bindsnet_b200.network.monitors import Monitor
     from oracle.oracle import OracleBackend
 
     spec = _draw(seed)
-    ref, x = _build(REF, spec)
-    rmon = {n: REF.monitors.Monitor(l, ["s"], time=spec["T"]) for n, l in ref.layers.items()}
-    for n, m in rmon.items():
-        ref.add_monitor(m, n)
-    ref.run(inputs={"X": x.clone()}, time=spec["T"])
 
+    def reference():
+        ref, x = _build(REF, spec)
+        rmon = {n: REF.monitors.Monitor(l, ["s"], time=spec["T"]) for n, l in ref.layers.items()}
+        for n, m in rmon.items():
+            ref.add_monitor(m, n)
+        ref.run(inputs={"X": x.clone()}, time=spec["T"])
+        counts = {n: m.get("s").reshape(spec["T"], spec["B"], -1).sum(0).numpy() for n, m in rmon.items()}
+        return _digest(x), counts, _snapshot(ref)
+
+    x_digest, ref_counts, a = stored("window", reference)
     ours, x2 = _build(cases.namespace("b200"), spec)
-    assert torch.equal(x, x2)
+    assert _digest(x2) == x_digest            # same input raster, drawn from the same seeded generator
     for n, l in ours.layers.items():
         ours.add_monitor(Monitor(l, ["s"], time=spec["T"]), n)
     with OracleBackend() as ob:
         ours.run(inputs={"X": x2}, time=spec["T"])
         assert ob.err == 0
 
-    a, b = _snapshot(ref), _snapshot(ours)
+    b = _snapshot(ours)
     assert a.keys() == b.keys(), (sorted(a), sorted(b))
     what = f"seed {seed} {spec['kind']} {spec['rule']} B={spec['B']}"
-    for n in ref.layers:   # spike counts per neuron over the window, exactly
-        ca = rmon[n].get("s").reshape(spec["T"], spec["B"], -1).sum(0).numpy()
+    for n, ca in ref_counts.items():   # spike counts per neuron over the window, exactly
         cb = ours.monitors[n].get("s").reshape(spec["T"], spec["B"], -1).sum(0).cpu().numpy()
         assert np.array_equal(ca, cb), f"{what}: spike counts of {n} differ"
     for k in a:

@@ -1,5 +1,5 @@
 """Pins the oracle (oracle/snn_oracle.c) against the LIVE reference: every fixture under
-tests/golden/ was produced by running /root/reference itself (gen_golden.py).  CPU only."""
+tests/golden/ was produced by running the original package itself (gen_golden.py).  CPU only."""
 import numpy as np
 import pytest
 

@@ -2,8 +2,9 @@
 ``bindsnet.models.DiehlAndCook2015`` (MulticompartmentConnection + Weight + MCC PostPre) and a classic
 ``Connection`` + ``learning.PostPre`` network — is described through ``include/snn_b200.h`` by
 ``bindsnet_b200.reference_binding`` (no bindsnet_b200 host classes) and run by the oracle library on the CPU; the
-result must equal what the reference's own ``Network.run`` computes on a twin network.  Skipped where the reference is
-not present (it is at /root/reference in the build container and under baseline/_ref after baseline/install_ref.sh)."""
+result must equal what the reference's own ``Network.run`` computes on a twin network.  These tests need the original
+package itself (stored results cannot stand in for its objects), so they skip unless it is importable: a checkout named
+by ``BINDSNET_REFERENCE``, or the install baseline/install_ref.sh makes under baseline/_ref (never part of a checkout)."""
 import os
 import sys
 

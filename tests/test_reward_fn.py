@@ -1,8 +1,8 @@
 """``Network(reward_fn=...)`` (reference: network.py:114-117, 325-326; learning/reward.py): the reward a window's
 MSTDP kernels are launched with is the reward_fn's ``compute`` of the run's kwargs.  Three episodes of a dense MSTDP
-network with ``MovingAvgRPE`` through the LIVE reference and through our host API on the oracle: same prediction
-state, same spikes, weights within the north_star's 1e-4.  CPU only; a GPU twin runs the same episodes on the kernels
-against the oracle bit for bit
+network with ``MovingAvgRPE`` through the reference (its results stored under tests/golden/live) and through our host
+API on the oracle: same prediction state, same spikes, weights within the north_star's 1e-4.  CPU only; a GPU twin runs
+the same episodes on the kernels against the oracle bit for bit
 (tests/test_zz_gpu_late_additions.py)."""
 import importlib
 
@@ -12,12 +12,7 @@ import torch
 
 import cases
 import helpers
-
-try:
-    REF = cases.namespace("reference")
-    REF_REWARD = importlib.import_module("bindsnet.learning.reward")
-except Exception:  # pragma: no cover
-    REF = None
+from live import REF, stored
 
 T, B = 60, 3
 REWARDS = (0.9, -0.4, 1.3)
@@ -49,13 +44,16 @@ def _plain_run(net, x, r):
     net.run(inputs={"X": x}, time=T, reward=r, a_plus=0.9, a_minus=-1.1)
 
 
-@pytest.mark.skipif(REF is None, reason="live reference not available")
 def test_reward_fn_matches_live_reference():
     from bindsnet_b200.learning.reward import MovingAvgRPE
     from oracle.oracle import OracleBackend
 
-    ref, xs = _net(REF, REF_REWARD.MovingAvgRPE)
-    seen_ref = _episodes(ref, [x.clone() for x in xs], _plain_run)
+    def reference():
+        ref, xs = _net(REF, importlib.import_module("bindsnet.learning.reward").MovingAvgRPE)
+        seen = _episodes(ref, [x.clone() for x in xs], _plain_run)
+        return seen, ref.layers["Y"].s, ref.connections[("X", "Y")].w.detach()
+
+    seen_ref, s_ref, w_ref = stored("episodes", reference)
 
     ours, xs2 = _net(cases.namespace("b200"), MovingAvgRPE)
     assert isinstance(ours.reward_fn, MovingAvgRPE)
@@ -65,8 +63,8 @@ def test_reward_fn_matches_live_reference():
 
     assert seen == seen_ref, (seen, seen_ref)                      # same fp32 arithmetic: equal, not close
     assert seen[0][0] != 0.0 and len(ours.reward_fn.rewards_predict_episode) == len(REWARDS)
-    assert np.array_equal(ref.layers["Y"].s.numpy(), ours.layers["Y"].s.numpy())
-    wa = ref.connections[("X", "Y")].w.detach().numpy()
+    assert np.array_equal(s_ref.numpy(), ours.layers["Y"].s.numpy())
+    wa = w_ref.numpy()
     wb = ours.connections[("X", "Y")].w.detach().numpy()
     assert np.abs(wa - wb).max() > -1 and not (np.abs(wa - wb) > 2e-6 + 1e-4 * np.abs(wa)).any(), np.abs(wa - wb).max()
     # the reward_fn changed what was learnt: the same episodes without it end elsewhere

@@ -1,11 +1,11 @@
-"""Run kwargs of ``Network.run`` that no golden fixture covers, through the LIVE reference and through our host API on
-the oracle, plus the kernels' CUDA sources on the emulation of tests/emu:
+"""Run kwargs of ``Network.run`` that no golden fixture covers, through the reference (its results stored under
+tests/golden/live) and through our host API on the oracle, plus the kernels' CUDA sources on the emulation of tests/emu:
 
 * ``a_plus`` / ``a_minus`` as dicts keyed by connection (network.py:359-377, 440-461): each connection's MSTDP sees its
   own entry, a connection without one the rule's defaults (learning.py:1552-1553);
 * ``clamp`` / ``unclamp`` as per-step INDEX tensors ``[T, k]`` (network.py:416-429), not only bool masks.
 
-CPU only; skipped where the reference is absent."""
+CPU only."""
 import os
 import sys
 
@@ -15,15 +15,10 @@ import torch
 
 import cases
 import helpers
+from live import REF, stored
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "emu"))
 
-try:
-    REF = cases.namespace("reference")
-except Exception:  # pragma: no cover
-    REF = None
-
-pytestmark = pytest.mark.skipif(REF is None, reason="live reference not available")
 T, B = 50, 2
 
 
@@ -57,8 +52,8 @@ def _clamped(ns):
     return net, x, {"clamp": {"Y": clamp}, "unclamp": {"Y": unclamp, "X": static}}
 
 
-def _compare(ref, ours, what):
-    a, b = helpers.snapshot(ref), helpers.snapshot(ours)
+def _compare(a, ours, what):
+    b = helpers.snapshot(ours)
     assert a.keys() == b.keys()
     for k in a:
         if k.endswith("/s"):
@@ -74,8 +69,12 @@ KW = {"reward": 0.6, "a_plus": {("X", "Y"): 0.7, ("Y", "Z"): 1.4}, "a_minus": {(
 def test_per_connection_a_plus_a_minus_match_the_live_reference():
     from oracle.oracle import OracleBackend
 
-    ref, x = _two_mstdp(REF)
-    ref.run(inputs={"X": x.clone()}, time=T, **{k: (dict(v) if isinstance(v, dict) else v) for k, v in KW.items()})
+    def reference():
+        ref, x = _two_mstdp(REF)
+        ref.run(inputs={"X": x.clone()}, time=T, **{k: (dict(v) if isinstance(v, dict) else v) for k, v in KW.items()})
+        return helpers.snapshot(ref)
+
+    ref = stored("state", reference)
     ours, x2 = _two_mstdp(cases.namespace("b200"))
     with OracleBackend() as ob:
         ours.run(inputs={"X": x2}, time=T, **KW)
@@ -91,16 +90,19 @@ def test_per_connection_a_plus_a_minus_match_the_live_reference():
 def test_per_step_index_clamps_match_the_live_reference():
     from oracle.oracle import OracleBackend
 
-    ref, x, kw = _clamped(REF)
-    rm = REF.monitors.Monitor(ref.layers["Y"], ["s"], time=T); ref.add_monitor(rm, "Y")
-    ref.run(inputs={"X": x.clone()}, time=T, **kw)
+    def reference():
+        ref, x, kw = _clamped(REF)
+        rm = REF.monitors.Monitor(ref.layers["Y"], ["s"], time=T); ref.add_monitor(rm, "Y")
+        ref.run(inputs={"X": x.clone()}, time=T, **kw)
+        return helpers.snapshot(ref), rm.get("s").reshape(T, B, -1).sum(dim=(0, 1)).numpy()
+
+    ref, ca = stored("state", reference)
     ours, x2, kw2 = _clamped(cases.namespace("b200"))
     helpers.add_spike_monitors(ours, T)
     with OracleBackend() as ob:
         ours.run(inputs={"X": x2}, time=T, **kw2)
         assert ob.err == 0
     _compare(ref, ours, "index clamps")
-    ca = rm.get("s").reshape(T, B, -1).sum(dim=(0, 1)).numpy()
     assert np.array_equal(ca, helpers.spike_counts(ours, T)["L/Y/count"])
     assert ca.sum() >= T      # the clamps fired
 

@@ -1,20 +1,16 @@
 """``SRM0Nodes`` (reference: nodes.py:1555-1701) on the scripted tier: with torch's generator seeded alike, a learning
-window of ``Input -> SRM0Nodes`` (PostPre, normalize) equals the live reference's — same spikes, voltages and weights
+window of ``Input -> SRM0Nodes`` (PostPre, normalize) equals the reference's — same spikes, voltages and weights
 within the north_star's tolerances (the built-in pieces run on the oracle backend here).  Also here, on the same tier:
-``learning.Rmax`` (the rule made for SRM0 targets) and ``IzhikevichNodes``.  CPU only."""
+``learning.Rmax`` (the rule made for SRM0 targets) and ``IzhikevichNodes``.  The reference's results are stored under
+tests/golden/live (see tests/golden/live.py).  CPU only."""
 import numpy as np
 import pytest
 import torch
 
 import cases
 import helpers
+from live import REF, stored
 
-try:
-    REF = cases.namespace("reference")
-except Exception:  # pragma: no cover
-    REF = None
-
-pytestmark = pytest.mark.skipif(REF is None, reason="live reference not available")
 T, B = 80, 3
 
 
@@ -35,11 +31,14 @@ def _net(ns, lbound=None):
 def test_srm0_window_matches_the_live_reference(lbound):
     from oracle.oracle import OracleBackend
 
-    ref, x = _net(REF, lbound)
-    rm = REF.monitors.Monitor(ref.layers["Y"], ["s", "v"], time=T); ref.add_monitor(rm, "Y")
-    torch.manual_seed(2024)
-    ref.run(inputs={"X": x.clone()}, time=T)
+    def reference():
+        ref, x = _net(REF, lbound)
+        rm = REF.monitors.Monitor(ref.layers["Y"], ["s", "v"], time=T); ref.add_monitor(rm, "Y")
+        torch.manual_seed(2024)
+        ref.run(inputs={"X": x.clone()}, time=T)
+        return rm.get("s"), rm.get("v"), helpers.snapshot(ref)
 
+    rs, rv, a = stored("window", reference)
     ours, x2 = _net(cases.namespace("b200"), lbound)
     assert ours._scripted_required()
     om = cases.namespace("b200").monitors.Monitor(ours.layers["Y"], ["s", "v"], time=T); ours.add_monitor(om, "Y")
@@ -47,9 +46,9 @@ def test_srm0_window_matches_the_live_reference(lbound):
     with OracleBackend() as ob:
         ours.run(inputs={"X": x2}, time=T)
         assert ob.err == 0
-    assert torch.equal(rm.get("s"), om.get("s")) and int(rm.get("s").sum()) > 20
-    assert torch.allclose(rm.get("v"), om.get("v"), rtol=1e-5, atol=1e-4)
-    a, b = helpers.snapshot(ref), helpers.snapshot(ours)
+    assert torch.equal(rs, om.get("s")) and int(rs.sum()) > 20
+    assert torch.allclose(rv, om.get("v"), rtol=1e-5, atol=1e-4)
+    b = helpers.snapshot(ours)
     assert a.keys() == b.keys()
     for k in a:
         if k.endswith("/s"):
@@ -78,10 +77,15 @@ def test_rmax_on_srm0_matches_the_live_reference():
         xs = [torch.bernoulli(0.3 * torch.ones(50, 1, 30), generator=g).byte() for _ in range(3)]
         return net, xs
 
-    ref, xs = build(REF)
-    torch.manual_seed(99)
-    for r, x in zip((1.0, -0.5, 0.8), xs):
-        ref.run(inputs={"X": x.clone()}, time=50, reward=r)
+    def reference():
+        ref, xs = build(REF)
+        torch.manual_seed(99)
+        for r, x in zip((1.0, -0.5, 0.8), xs):
+            ref.run(inputs={"X": x.clone()}, time=50, reward=r)
+        Y, c = ref.layers["Y"], ref.connections[("X", "Y")]
+        return Y.s, Y.v, c.w.detach(), c.update_rule.eligibility_trace
+
+    rs, rv, wa, ea = stored("windows", reference)
     ours, xs2 = build(cases.namespace("b200"))
     assert ours._scripted_required()
     torch.manual_seed(99)
@@ -89,11 +93,11 @@ def test_rmax_on_srm0_matches_the_live_reference():
         for r, x in zip((1.0, -0.5, 0.8), xs2):
             ours.run(inputs={"X": x}, time=50, reward=r)
         assert ob.err == 0
-    assert torch.equal(ref.layers["Y"].s, ours.layers["Y"].s)
-    assert torch.allclose(ref.layers["Y"].v, ours.layers["Y"].v, rtol=1e-5, atol=1e-4)
-    wa, wb = ref.connections[("X", "Y")].w.detach(), ours.connections[("X", "Y")].w.detach()
+    assert torch.equal(rs, ours.layers["Y"].s)
+    assert torch.allclose(rv, ours.layers["Y"].v, rtol=1e-5, atol=1e-4)
+    wb = ours.connections[("X", "Y")].w.detach()
     assert not ((wa - wb).abs() > 2e-6 + 1e-4 * wa.abs()).any(), float((wa - wb).abs().max())
-    ea, eb = ref.connections[("X", "Y")].update_rule.eligibility_trace, ours.connections[("X", "Y")].update_rule.eligibility_trace
+    eb = ours.connections[("X", "Y")].update_rule.eligibility_trace
     assert torch.allclose(ea, eb, rtol=1e-4, atol=1e-5) and float(eb.abs().sum()) > 0
 
 
@@ -114,19 +118,27 @@ def test_izhikevich_nodes_match_the_live_reference(excitatory):
                                                   nu=(1e-3, 1e-2), reduction=torch.sum, wmin=0.0, wmax=8.0), "X", "Y")
         return net, torch.bernoulli(0.3 * torch.ones(70, 2, 30), generator=g).byte()
 
-    ref, x = build(REF)
+    params = ("r", "a", "b", "c", "d", "S", "excitatory", "u")
+    state = ("v", "u", "x", "summed")
+
+    def reference():
+        ref, x = build(REF)
+        built = {name: getattr(ref.layers["Y"], name).clone() for name in params}
+        rm = REF.monitors.Monitor(ref.layers["Y"], ["s"], time=70); ref.add_monitor(rm, "Y")
+        ref.run(inputs={"X": x.clone()}, time=70)
+        return built, rm.get("s"), {name: getattr(ref.layers["Y"], name) for name in state}, ref.connections[("X", "Y")].w.detach()
+
+    built, rs, after, wa = stored("window", reference)
     ours, x2 = build(cases.namespace("b200"))
-    for name in ("r", "a", "b", "c", "d", "S", "excitatory", "u"):
-        assert torch.equal(getattr(ref.layers["Y"], name), getattr(ours.layers["Y"], name)), name
-    rm = REF.monitors.Monitor(ref.layers["Y"], ["s"], time=70); ref.add_monitor(rm, "Y")
+    for name in params:
+        assert torch.equal(built[name], getattr(ours.layers["Y"], name)), name
     om = cases.namespace("b200").monitors.Monitor(ours.layers["Y"], ["s"], time=70); ours.add_monitor(om, "Y")
-    ref.run(inputs={"X": x.clone()}, time=70)
     assert ours._scripted_required()
     with OracleBackend() as ob:
         ours.run(inputs={"X": x2}, time=70)
         assert ob.err == 0
-    assert torch.equal(rm.get("s"), om.get("s")) and int(om.get("s").sum()) > 10
-    for name in ("v", "u", "x", "summed"):
-        assert torch.allclose(getattr(ref.layers["Y"], name), getattr(ours.layers["Y"], name), rtol=1e-4, atol=1e-3), name
-    wa, wb = ref.connections[("X", "Y")].w.detach(), ours.connections[("X", "Y")].w.detach()
+    assert torch.equal(rs, om.get("s")) and int(om.get("s").sum()) > 10
+    for name in state:
+        assert torch.allclose(after[name], getattr(ours.layers["Y"], name), rtol=1e-4, atol=1e-3), name
+    wb = ours.connections[("X", "Y")].w.detach()
     assert not ((wa - wb).abs() > 2e-6 + 1e-4 * wa.abs()).any(), float((wa - wb).abs().max())
